@@ -101,6 +101,26 @@ class ClockSampler(threading.Thread):
                 "samples": len(sm)}
 
 
+def dump_outputs(cf, out_dir, max_rows=1 << 18):
+    """What a caller of processFrame reads back after the last timed step, as DIR/<name>.npy: every model's pose
+    and tracking statistics, and the camera model's surfel map (a fixed, seeded sample of max_rows rows when it
+    is larger, so that the files stay small)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = cf.num_models
+    stats = [cf.last_stats(i) for i in range(n)]
+    surfels = cf.model(0).download_map()
+    count = len(surfels)
+    if count > max_rows:
+        surfels = surfels[np.sort(np.random.default_rng(0).choice(count, max_rows, replace=False))]
+    out = {"poses": np.stack([cf.pose(i) for i in range(n)]).astype(np.float32),
+           "track_stats": np.array([[s.lastICPError, s.lastICPCount, s.lastRGBError, s.lastRGBCount, s.lastSO3Error,
+                                     s.lastSO3Count] for s in stats], np.float64),
+           "surfel_count": np.array([count], np.float64),
+           "surfels": surfels.astype(np.float32)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_port_fps(frames, n_frames, warm=2):
     """The CPU restatement of the same per-frame path (oracle/, single thread) on a bounded sample."""
     from orc_pipeline import OraclePipeline
@@ -237,6 +257,7 @@ def main():
     ap.add_argument("--impl", default="cofusion_b200")
     ap.add_argument("--cpu-frames", type=int, default=8, help="frames of the cpu_baseline sample (0 = skip)")
     ap.add_argument("--objects-steps", type=int, default=300, help="steps of the configs[2] leg at N = 1 (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         # the reference's path on the host cores: a bounded sample of the K requested steps (run_reference)
@@ -293,7 +314,7 @@ def main():
 
     keep = []
 
-    def timed(frames, sampler=None):
+    def timed(frames, sampler=None, dump_dir=None):
         cf = build()
         keep.append(cf)
         ext = torch.cuda.ExternalStream(cf.ctx.stream)  # only used to record / wait on events
@@ -325,6 +346,8 @@ def main():
         if sampler:
             sampler.stop_flag = True
         launches = cf.ctx.take_launch_count()
+        if dump_dir and rank == 0:
+            dump_outputs(cf, dump_dir)
         # the tracker kernel is timed with CUDA events on its own stream: every launch of a short extra run (the
         # event pair is read back per launch, which would serialise the timed region above)
         ksum, kn = 0.0, 0
@@ -341,7 +364,7 @@ def main():
         return float(t_ms.item()), launches, (ksum, kn), nsurf, mine
 
     sampler = ClockSampler(local) if rank == 0 else None
-    ms, launches, (kms, kn), nsurf, mine = timed(devf, sampler)
+    ms, launches, (kms, kn), nsurf, mine = timed(devf, sampler, args.dump_outputs)
     ms_e2e, _, _, _, _ = timed(host)
     if rank != 0:
         # done: the reductions inside timed() were the last collectives.  Leave without a rank-by-rank tear-down of

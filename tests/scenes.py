@@ -1,5 +1,6 @@
 """Seeded tracker test cases shared by CPU and GPU tests."""
 import functools
+import hashlib
 
 import numpy as np
 
@@ -71,3 +72,24 @@ def nan_equal(a, b, tol=0.0, ref_plane_rows=None):
         return ok, "max abs diff %g" % (np.abs(a[m] - b[m]).max() if m.any() else 0)
     d = np.abs(a[m] - b[m]).max() if m.any() else 0.0
     return d <= tol, "max abs diff %g" % d
+
+
+def digest(a):
+    """SHA-256 of an array's bytes, every NaN replaced by one canonical NaN (equal_nan semantics)"""
+    a = np.ascontiguousarray(a).copy()
+    if a.dtype.kind == "f":
+        a[np.isnan(a)] = np.nan
+    return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+def nan_digest(a):
+    """SHA-256 of an array's NaN pattern"""
+    return hashlib.sha256(np.packbits(np.isnan(a)).tobytes()).hexdigest()
+
+
+def case_digest(case):
+    """fingerprint of the inputs of a room_pair case"""
+    h = hashlib.sha256()
+    for k in ("d0", "rgb0", "T0", "d1", "rgb1", "v4", "n4", "img"):
+        h.update(np.ascontiguousarray(case[k]).tobytes())
+    return h.hexdigest()

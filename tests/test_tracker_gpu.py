@@ -1,6 +1,7 @@
 """-m gpu: parity of the CUDA tracker path (through the C ABI) against
    (1) the CPU oracle (oracle/tracker.c) and
-   (2) the reference's own CUDA kernels compiled for sm_100a (oracle/_ref/libcfref.so), when built.
+   (2) the reference's own CUDA kernels compiled for sm_100a, through their outputs on the same inputs
+       (tests/golden/tracker_ref_cases_sm100a.npz, made by tests/golden/make_ref_cases.py).
 
 Tolerances (north_star: 1e-4 relative on float buffers, bit-exact on integer/index work):
   - integer outputs (grey, gradients, u8 pyramids, correspondence flags/counts): bit-exact vs oracle
@@ -9,6 +10,8 @@ Tolerances (north_star: 1e-4 relative on float buffers, bit-exact on integer/ind
   - reduction sums A, b: <= 1e-4 relative (f32 tree sums vs f64 oracle sums)
   - poses: <= 1e-4 absolute on R and t
 """
+import os
+
 import numpy as np
 import pytest
 
@@ -18,12 +21,39 @@ import scenes
 pytestmark = pytest.mark.gpu
 
 ANGLE = float(np.sin(np.deg2rad(20.0)))
+REF_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "tracker_ref_cases_sm100a.npz")
 
 
 @pytest.fixture(scope="module")
 def gu():
     import gpu_util
     return gpu_util
+
+
+@pytest.fixture(scope="module")
+def ref_golden():
+    return dict(np.load(REF_GOLDEN))
+
+
+def _ref_outputs(ref_golden, case):
+    """the reference kernels' outputs for this case, keyed by name"""
+    p = "c%dx%d_" % (case["W"], case["H"])
+    assert str(ref_golden[p + "inputs"]) == scenes.case_digest(case), (
+        "room_pair(%d, %d) no longer renders the inputs the stored reference outputs were computed from: "
+        "regenerate them with tests/golden/make_ref_cases.py" % (case["W"], case["H"]))
+    return {k[len(p):]: v for k, v in ref_golden.items() if k.startswith(p)}
+
+
+def _check_sampled(r, name, x, planes, tol, scaled=True):
+    """planar image x against the reference's: NaN pattern of the first plane, then every plane at the stored
+    pixels within tol (times max(1, max |value|) of the reference's plane when scaled)"""
+    h = x.shape[0] // planes
+    assert scenes.nan_digest(x[:h]) == str(r[name + "_nan"]), "%s: NaN pattern differs from the reference" % name
+    idx = r[name + "_idx"]
+    for k in range(planes):
+        d = np.abs(x[k * h:(k + 1) * h].reshape(-1)[idx] - r[name + "_val"][k]).max()
+        lim = tol * (max(1.0, float(r[name + "_absmax"][k])) if scaled else 1.0)
+        assert d <= lim, "%s plane %d: max abs diff %g > %g" % (name, k, d, lim)
 
 
 @pytest.fixture(scope="module", params=[(640, 480), (160, 120), (72, 52)], ids=["640x480", "160x120", "72x52"])
@@ -75,45 +105,29 @@ def test_image_preparation_matches_oracle(gu, case):
     assert np.array_equal(orc.project_cloud(vd, K), gu.project_cloud(vd, K), equal_nan=True)
 
 
-def test_image_preparation_matches_reference_kernels(gu, case):
-    ref = orc.ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/libcfref.so not built (needs /root/reference at build time)")
+def test_image_preparation_matches_reference_kernels(gu, case, ref_golden):
+    r = _ref_outputs(ref_golden, case)
     K = case["K"]
     df = orc.bilateral(case["d1"], 5.0)
     # the reference build contracts to FMA and uses approximate division: last-ulp differences
-    pr, pg = orc.pyr_down_f(df, ref), gu.pyr_down_f(df)
-    assert np.array_equal(np.isnan(pr), np.isnan(pg)) and np.nanmax(np.abs(pr - pg)) <= 2e-6 * np.nanmax(np.abs(pr))
+    _check_sampled(r, "pyr_f", gu.pyr_down_f(df), 1, 2e-6)
     g = orc.rgb_to_intensity(case["rgb1"])
-    assert np.array_equal(orc.pyr_down_u8(g, ref), gu.pyr_down_u8(g))
-    dx_r, dy_r = orc.derivative_images(g, ref)
+    assert scenes.digest(gu.pyr_down_u8(g)) == str(r["pyr_u8"])
+    # the reference's gradients are stored as the pixels where they differ from the oracle's
+    dx_r, dy_r = orc.derivative_images(g)
+    dx_r.reshape(-1)[r["dx_idx"]] = r["dx_val"]
+    dy_r.reshape(-1)[r["dy_idx"]] = r["dy_val"]
     dx_g, dy_g = gu.derivative_images(g)
     # the reference build contracts a*b+c into FMA: a 1-LSB flip at an exact .0 boundary is possible
     assert np.abs(dx_r.astype(int) - dx_g.astype(int)).max() <= 1 and (dx_r != dx_g).mean() < 1e-3
     assert np.abs(dy_r.astype(int) - dy_g.astype(int)).max() <= 1 and (dy_r != dy_g).mean() < 1e-3
-    v_r, v_g = orc.create_vmap(df, K, 20.0, ref), gu.create_vmap(df, K, 20.0)
-    m = ~np.isnan(v_r[:case["H"]])
-    assert np.array_equal(np.isnan(v_r[:case["H"]]), np.isnan(v_g[:case["H"]]))
-    for k in range(3):
-        pr, pg = v_r[k * case["H"]:(k + 1) * case["H"]][m], v_g[k * case["H"]:(k + 1) * case["H"]][m]
-        assert np.abs(pr - pg).max() <= 2e-6 * max(1.0, np.abs(pr).max())
-    n_r, n_g = orc.create_nmap(v_g, ref), gu.create_nmap(v_g)
-    H = case["H"]
-    m = ~np.isnan(n_r[:H])
-    assert np.array_equal(np.isnan(n_r[:H]), np.isnan(n_g[:H]))
-    for k in range(3):
-        assert np.abs(n_r[k * H:(k + 1) * H][m] - n_g[k * H:(k + 1) * H][m]).max() <= 5e-6
-    cv_r, cn_r = orc.copy_maps(case["v4"], case["n4"], ref)
+    v_g = gu.create_vmap(df, K, 20.0)
+    _check_sampled(r, "vmap", v_g, 3, 2e-6)
+    _check_sampled(r, "nmap", gu.create_nmap(v_g), 3, 5e-6, scaled=False)
     cv_g, cn_g = gu.copy_maps(case["v4"], case["n4"])
-    assert scenes.nan_equal(cv_g, cv_r)[0] and scenes.nan_equal(cn_g, cn_r)[0]
-    rv_r, rv_g = orc.resize_map(cv_r, False, ref), gu.resize_map(cv_r, False)
-    m = ~np.isnan(rv_r[:H // 2])
-    assert np.array_equal(np.isnan(rv_r[:H // 2]), np.isnan(rv_g[:H // 2]))
-    for k in range(3):
-        a, b = rv_r[k * (H // 2):(k + 1) * (H // 2)][m], rv_g[k * (H // 2):(k + 1) * (H // 2)][m]
-        assert np.abs(a - b).max() <= 2e-6 * max(1.0, np.abs(a).max())
-    vd_r, vd_g = orc.vertices_to_depth(case["v4"], 6.0, ref), gu.vertices_to_depth(case["v4"], 6.0)
-    assert np.array_equal(vd_r, vd_g, equal_nan=True)
+    assert scenes.digest(cv_g) == str(r["copy_v"]) and scenes.digest(cn_g) == str(r["copy_n"])
+    _check_sampled(r, "resize_v", gu.resize_map(cv_g, False), 3, 2e-6)
+    assert scenes.digest(gu.vertices_to_depth(case["v4"], 6.0)) == str(r["v2d"])
 
 
 def _step_inputs(case, level, perturb=True):
@@ -132,11 +146,12 @@ def _step_inputs(case, level, perturb=True):
 
 
 @pytest.mark.parametrize("level", [0, 1, 2])
-def test_reduction_steps_match_oracle_and_reference(gu, case, level):
+def test_reduction_steps_match_oracle_and_reference(gu, case, level, ref_golden):
     if case["W"] < 160 and level > 0:
         pytest.skip("tiny case: level 0 only")
     od, Kl, v, dx, dy, cloud, T0, T = _step_inputs(case, level)
-    ref = orc.ref()
+    r = _ref_outputs(ref_golden, case)
+    q = "L%d_" % level
     Rpi = np.linalg.inv(T0[:3, :3]).astype(np.float32)
     args = (T[:3, :3], T[:3, 3], v[0], v[1], Rpi, T0[:3, 3], Kl, v[2], v[3], 0.10, ANGLE)
     # ---- ICP
@@ -149,10 +164,9 @@ def test_reduction_steps_match_oracle_and_reference(gu, case, level):
     assert np.allclose(A_g, A_g.T)
     diff = np.abs(e_g - e_o)
     assert (diff > 1e-5).mean() < 1e-3  # borderline association flips only
-    if ref is not None:
-        A_r, b_r, r_r, _ = orc.icp_step(*args, lib=ref)
-        assert abs(r_g[1] - r_r[1]) <= max(2, 2e-4 * r_r[1])
-        assert scenes.relerr(A_g, A_r) < 1e-4 and scenes.relerr(b_g, b_r) < 1e-4
+    A_r, b_r, r_r = r[q + "icp_A"], r[q + "icp_b"], r[q + "icp_res"]
+    assert abs(r_g[1] - r_r[1]) <= max(2, 2e-4 * r_r[1])
+    assert scenes.relerr(A_g, A_r) < 1e-4 and scenes.relerr(b_g, b_r) < 1e-4
     # ---- RGB residual
     T_rel = np.linalg.inv(T) @ T0  # any small relative motion
     krk, kt = scenes.warp_for(Kl, T_rel)
@@ -167,24 +181,22 @@ def test_reduction_steps_match_oracle_and_reference(gu, case, level):
     both = vo & vg
     assert ((zxo[both] != zxg[both]) | (zyo[both] != zyg[both])).mean() < 1e-3
     assert abs(n_g - n_o) <= max(2, 1e-3 * n_o) and abs(s_g - s_o) <= max(2000, 2e-3 * abs(s_o))
-    if ref is not None:
-        c_r, s_r, n_r = orc.rgb_residual(minScale, dx, dy, v[4], v[5], v[6], v[7], 0.07, kt, krk, lib=ref)
-        assert abs(n_g - n_r) <= max(2, 1e-3 * n_r) and abs(s_g - s_r) <= max(2000, 2e-3 * abs(s_r))
+    s_r, n_r = int(r[q + "res_sigma"]), int(r[q + "res_count"])
+    assert abs(n_g - n_r) <= max(2, 1e-3 * n_r) and abs(s_g - s_r) <= max(2000, 2e-3 * abs(s_r))
     # ---- RGB step on identical correspondences
     sigma = float(n_o)
     A_o, b_o = orc.rgb_step(c_o, sigma, cloud, Kl, dx, dy, 0.125)
     A_g, b_g = gu.rgb_step(c_o, sigma, cloud, Kl, dx, dy, 0.125)
     assert scenes.relerr(A_g, A_o) < 1e-4 and scenes.relerr(b_g, b_o) < 1e-4
-    if ref is not None:
-        A_r, b_r = orc.rgb_step(c_o, sigma, cloud, Kl, dx, dy, 0.125, lib=ref)
-        assert scenes.relerr(A_g, A_r) < 1e-4 and scenes.relerr(b_g, b_r) < 1e-4
+    A_r, b_r = r[q + "rgb_A"], r[q + "rgb_b"]
+    assert scenes.relerr(A_g, A_r) < 1e-4 and scenes.relerr(b_g, b_r) < 1e-4
     # rgbOnly signalling (sigma == -1 -> unit weights)
     A_o1, b_o1 = orc.rgb_step(c_o, -1.0, cloud, Kl, dx, dy, 0.125)
     A_g1, b_g1 = gu.rgb_step(c_o, -1.0, cloud, Kl, dx, dy, 0.125)
     assert scenes.relerr(A_g1, A_o1) < 1e-4 and scenes.relerr(b_g1, b_o1) < 1e-4
 
 
-def test_so3_step_matches_oracle_and_reference(gu, case):
+def test_so3_step_matches_oracle_and_reference(gu, case, ref_golden):
     if case["W"] < 160:
         pytest.skip("so3 runs on level 2")
     od, df = scenes.oracle_odometry(case)
@@ -198,10 +210,9 @@ def test_so3_step_matches_oracle_and_reference(gu, case):
     A_g, b_g, r_g = gu.so3_step(last, nxt, H_, Kinv, KR)
     assert r_o[1] > 100 and r_g[1] == r_o[1]
     assert scenes.relerr(A_g, A_o) < 1e-4 and scenes.relerr(b_g, b_o) < 1e-4 and abs(r_g[0] - r_o[0]) <= 1e-4 * r_o[0]
-    ref = orc.ref()
-    if ref is not None:
-        A_r, b_r, r_r = orc.so3_step(last, nxt, H_, Kinv, KR, lib=ref)
-        assert r_g[1] == r_r[1] and scenes.relerr(A_g, A_r) < 1e-4 and scenes.relerr(b_g, b_r) < 1e-4
+    r = _ref_outputs(ref_golden, case)
+    A_r, b_r, r_r = r["so3_A"], r["so3_b"], r["so3_res"]
+    assert r_g[1] == r_r[1] and scenes.relerr(A_g, A_r) < 1e-4 and scenes.relerr(b_g, b_r) < 1e-4
 
 
 def _cuda_odometry(gu, case, cutoff=20.0, maxD=5.0):
@@ -220,7 +231,7 @@ def _cuda_odometry(gu, case, cutoff=20.0, maxD=5.0):
 
 
 @pytest.mark.parametrize("variant", ["persistent", "per_step_kernels", "host_loop"])
-def test_full_tracking_matches_oracle(gu, case, variant):
+def test_full_tracking_matches_oracle(gu, case, variant, ref_golden):
     host_loop = variant == "host_loop"
     if case["W"] < 160:
         pytest.skip("pyramid needs >= 160x120")
@@ -251,10 +262,8 @@ def test_full_tracking_matches_oracle(gu, case, variant):
     eg = err_g.cpu().numpy()
     assert (np.abs(eg - err_o) > 1e-4).mean() < 2e-3
     # reference kernels driven through the same loop agree as well
-    if orc.ref() is not None:
-        oo2, _ = scenes.oracle_odometry(case)
-        p_r, st_r, _, extra = oo2.track(case["T0"], use_ref=True)
-        assert np.abs(p_g - p_r).max() < 1e-4, (p_g, p_r)
+    p_r = _ref_outputs(ref_golden, case)["track_pose"]
+    assert np.abs(p_g - p_r).max() < 1e-4, (p_g, p_r)
 
 
 def test_tracking_is_deterministic_and_flag_variants_agree(gu):
