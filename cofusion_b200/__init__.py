@@ -77,9 +77,6 @@ class Odometry:
             _lib.cfb_odom_destroy(self._h)
             self._h = C.c_void_p()
 
-    def set_mode(self, mode):
-        check(lib().cfb_odom_set_mode(self._h, int(mode)))
-
     def init_icp(self, depth_pyr, cutoff):
         ptrs = (C.c_void_p * 3)(*[d.data_ptr() for d in depth_pyr])
         pitch = (C.c_size_t * 3)(*[d.stride(0) * 4 for d in depth_pyr])
@@ -265,10 +262,6 @@ class Model:
         o.__class__ = type("BorrowedOdometry", (Odometry,), {"__del__": lambda self_: None})
         self.ctx.sync()
         return o.view(which, level)
-
-    def odometry_set_mode(self, mode):
-        lib().cfb_model_odometry.restype = C.c_void_p
-        check(lib().cfb_odom_set_mode(C.c_void_p(lib().cfb_model_odometry(self._h)), int(mode)))
 
     def initialise(self, time, max_depth=20.0):
         check(lib().cfb_model_initialise(self._h, int(time), C.c_float(max_depth)))

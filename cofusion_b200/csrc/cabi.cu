@@ -362,12 +362,6 @@ int cfb_odom_get_incremental_transformation(cfb_odom* o, float trans[3], float r
   if (stats_out) memcpy(stats_out, &o->impl.stats(), sizeof(cfb_track_stats));
   return 0;
 }
-int cfb_odom_set_mode(cfb_odom* o, int mode) {
-  REQUIRE(o && (mode == 0 || mode == 1), "odom_set_mode");
-  DevScope dev_scope__(device_of(o));
-  o->impl.setMode(mode);
-  return 0;
-}
 int cfb_odom_enable_kernel_timing(cfb_odom* o, int on) {
   REQUIRE(o, "odom_enable_kernel_timing");
   DevScope dev_scope__(device_of(o));

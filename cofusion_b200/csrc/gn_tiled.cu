@@ -33,15 +33,64 @@
 // Per-pixel arithmetic: SURVEY.md Appendix A1-A5 (tracker_device.cuh holds the stand-alone form).
 #include <cuda.h>  // CUtensorMap + enums only; the encoder is fetched through cudaGetDriverEntryPoint
 
+#include <float.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
-#include "gn_serial.cuh"
+#include "gn_math.h"
 #include "image_kernels.cuh"
+#include "odometry.cuh"
 #include "pose_math.cuh"
+#include "tracker_device.cuh"
 
 namespace cfb {
+namespace dev {
+
+struct LevelK {  // f32 level intrinsics (CameraModel::operator())
+  float fx, fy, cx, cy;
+};
+
+// RGBDOdometry.cpp:373-374
+__device__ __forceinline__ float rgb_sigma_from_counts(int cnt, int sg, float* tmpErrorOut) {
+  const float tmpError = (float)(sqrt((double)sg) / (double)cnt);
+  if (tmpErrorOut) *tmpErrorOut = tmpError;
+  return (tmpError == 0.f) ? 1.f : (float)cnt;
+}
+
+// ---- frame-side photometric preparation, once per level per frame: gradient images
+// (cudafuncs.cu:658-683) + every iteration-invariant gate of RGBResidual::getProducts folded into one
+// byte per pixel: j0 < W-5, i < H-1 (reduce.cu:799), 4x4 window of nextImage > 0 (:803-814),
+// gradient magnitude gate (:823-825), nextDepth not NaN (:832).
+__constant__ float c_sx[9] = {0.52201f, 0.00000f, -0.52201f, 0.79451f, -0.00000f, -0.79451f, 0.52201f, 0.00000f, -0.52201f};
+__constant__ float c_sy[9] = {0.52201f, 0.79451f, 0.52201f, 0.00000f, 0.00000f, 0.00000f, -0.52201f, -0.79451f, -0.52201f};
+__device__ __forceinline__ void rgb_prepare_pixel(const unsigned char* __restrict__ img, int W, int H,
+                                                  const float* __restrict__ nextDepth, float minScale,
+                                                  short* __restrict__ dx, short* __restrict__ dy,
+                                                  unsigned char* __restrict__ cand, int x, int y) {
+  float dxVal = 0.f, dyVal = 0.f;
+  int k = 8;
+  for (int j = max(y - 1, 0); j <= min(y + 1, H - 1); j++)
+    for (int i = max(x - 1, 0); i <= min(x + 1, W - 1); i++) {
+      float p = (float)__ldg(img + j * W + i);
+      dxVal = __fadd_rn(dxVal, __fmul_rn(p, c_sx[k]));  // no FMA contraction: bit-identical to
+      dyVal = __fadd_rn(dyVal, __fmul_rn(p, c_sy[k]));  // computeDerivativeImages in image_kernels.cu
+      --k;
+    }
+  const short sx = (short)dxVal, sy = (short)dyVal;
+  dx[y * W + x] = sx;
+  dy[y * W + x] = sy;
+  unsigned ok = (x < W - 5 && y < H - 1) ? 1u : 0u;
+  for (int u = max(y - 2, 0); u < min(y + 2, H); u++)
+    for (int v = max(x - 2, 0); v < min(x + 2, W); v++) ok &= (unsigned)(__ldg(img + u * W + v) > 0);
+  const float mTwo = (float)((sx * sx) + (sy * sy));
+  ok &= (unsigned)(mTwo >= minScale);
+  ok &= (unsigned)(!isnan(__ldg(nextDepth + y * W + x)));
+  cand[y * W + x] = (unsigned char)ok;
+}
+
+}  // namespace dev
+
 namespace {
 using namespace dev;
 
@@ -1023,7 +1072,7 @@ __device__ __noinline__ void gn_solve_warp(int m, int lvl_next, int is_last, flo
   __syncwarp();
 }
 
-// H = K R K^-1 etc. of the SO(3) step (gn_serial.cuh: so3_matrices), lane e < 9 owns element e
+// H = K R K^-1 etc. of the SO(3) step (as the host loop in odometry.cu), lane e < 9 owns element e
 __device__ __forceinline__ void so3_matrices_warp(GNState* g) {
   TSMEM();
   const int lane = threadIdx.x & 31;
@@ -1805,7 +1854,7 @@ cudaError_t RGBDOdometry::prepareTiled(int nm) {
 
 size_t RGBDOdometry::tiledScratchBytes() { return kSyncBytes + 256; }
 
-bool RGBDOdometry::canBatch(int n) const { return n >= 1 && n <= kMaxM && mode_ == 0 && width < 2048 && height < 2048; }
+bool RGBDOdometry::canBatch(int n) const { return n >= 1 && n <= kMaxM && width < 2048 && height < 2048; }
 
 cudaError_t RGBDOdometry::enqueuePrepare(cudaStream_t s, void* sync_words, int nmodels, bool extents) {
   PrepParams pp;
@@ -1959,7 +2008,6 @@ cudaError_t RGBDOdometry::trackTiled(RGBDOdometry* const* od, int n, float (*tra
       o.lastNextImage[i] = o.nextImage[i];
       o.nextImage[i] = t;
     }
-    o.parity_ ^= 1;
   };
   if (async) {  // the caller reads pose / stats later (device pose block, statsDevice()); nothing to wait for
     for (int m = 0; m < n; ++m) swap_so3_images(*od[m]);

@@ -58,7 +58,7 @@ RGBDOdometry::RGBDOdometry(int w, int h, float cx, float cy, float fx, float fy,
 }
 
 // Back to the state of a freshly constructed object (a pooled Model is handed to a new object id): every device
-// buffer the constructor zeroed is zeroed again on `s`; plans, graphs and tensor maps (tied to the buffers) stay.
+// buffer the constructor zeroed is zeroed again on `s`; plans and tensor maps (tied to the buffers) stay.
 cudaError_t RGBDOdometry::recycle(cudaStream_t s) {
   for (auto& z : zeroed_) RET_IF(cudaMemsetAsync(z.first, 0, z.second, s));
   memset(&stats_, 0, sizeof(stats_));
@@ -83,7 +83,6 @@ RGBDOdometry::~RGBDOdometry() {
     cudaFree(corresImg[i]);
     cudaFree(rgbCand[i]);
   }
-  for (auto& e : graphs_) cudaGraphExecDestroy(e.exec);
   cudaFree(d_pose_in);
   cudaFree(grid_sync_);
   cudaFree(tiled_scratch_);
@@ -228,8 +227,16 @@ cudaError_t RGBDOdometry::getIncrementalTransformation(float trans[3], float rot
                                                        cudaStream_t s) {
   bool icp = !rgbOnly && icpWeight > 0;
   bool rgb = rgbOnly || icpWeight < 100;
-  if (!force_host_loop && icp && rgb)
-    return deviceLoop(trans, rot, icpWeight, pyramid, fastOdom, so3, err, err_pitch, s);
+  if (!force_host_loop && icp && rgb) {
+    if (!tiled_scratch_) {
+      RET_IF(cudaMalloc(&tiled_scratch_, tiledScratchBytes()));
+      RET_IF(cudaMemsetAsync(tiled_scratch_, 0, tiledScratchBytes(), s));
+    }
+    RGBDOdometry* od[1] = {this};
+    float* errs[1] = {err};
+    return trackTiled(od, 1, (float(*)[3])trans, (float(*)[9])rot, icpWeight, pyramid, fastOdom, so3, errs, err_pitch,
+                      tiled_scratch_, s);
+  }
   return hostLoop(trans, rot, rgbOnly, icpWeight, pyramid, fastOdom, so3, err, err_pitch, s);
 }
 

@@ -5,12 +5,12 @@
 //     hot loop, reduce.cu:958, cudafuncs.cu:525/:581);
 //   * no cudaDeviceSynchronize inside: everything is enqueued on one stream.
 // Two execution paths for getIncrementalTransformation:
-//   HostLoop   - generic (all flag combinations): one fused launch per step, one stream sync + tiny
+//   HostLoop   - generic (all flag combinations); taken when ICP or RGB is off (rgbOnly, icpWeight <= 0
+//                or >= 100) or force_host_loop is set: one fused launch per step, one stream sync + tiny
 //                D2H per step, FP64 GN step on the host (gn_math.h).  Mirrors the reference loop 1:1.
-//   DeviceLoop - default flags (icp && rgb, no early exit): whole SO3 + 19-iteration GN sequence runs
-//                without host involvement; the FP64 GN step runs on the device.  Two realisations:
-//                mode 0 = ONE persistent cooperative kernel over shared-memory tiles (gn_tiled.cu, default),
-//                mode 1 = one fused kernel per step, captured in a CUDA graph (gn_device.cu).
+//   Persistent - ICP and RGB both on (the default flags): the whole SO3 + GN sequence is ONE persistent
+//                cooperative kernel over shared-memory tiles (gn_tiled.cu, trackTiled) that runs the FP64
+//                GN step on the device; the host reads back pose + stats once per frame.
 #pragma once
 #include <utility>
 #include <vector>
@@ -31,7 +31,7 @@ struct TrackStats {  // RGBDOdometry.h:62-70
   int pad;
 };
 
-// Device-resident Gauss-Newton state (DeviceLoop).
+// Device-resident Gauss-Newton state (persistent kernel).
 struct GNState {
   double resultRt[16];
   double resultR[9], lastResultR[9];
@@ -112,10 +112,6 @@ class RGBDOdometry {
                                unsigned char* const* destImages, cudaStream_t s);
   cudaError_t hostLoop(float trans[3], float rot[9], bool rgbOnly, float icpWeight, bool pyramid, bool fastOdom,
                        bool so3, float* err, size_t err_pitch, cudaStream_t s);
-  cudaError_t deviceLoop(float trans[3], float rot[9], float icpWeight, bool pyramid, bool fastOdom, bool so3,
-                         float* err, size_t err_pitch, cudaStream_t s);
-  cudaError_t enqueueDeviceLoop(float icpWeight, bool pyramid, bool fastOdom, bool so3, float* err,
-                                size_t err_pitch, cudaStream_t s);
   cudaError_t prepareTiled(int nmodels);
   void destroyTiled();
   std::vector<std::pair<void*, size_t>> zeroed_;  // device buffers the constructor zero-initialised
@@ -146,20 +142,6 @@ class RGBDOdometry {
   void* h_pinned;    // pinned staging for small H2D/D2H
   unsigned char* rgbCand[NUM_PYRS];  // iteration-invariant photometric gates, one byte per pixel
   float* d_pose_in;                  // t[3], R[9] of the incoming pose
-  struct GraphKey {
-    int parity;
-    float* err;
-    size_t err_pitch;
-    float icpWeight;
-    bool pyramid, fastOdom, so3;
-  };
-  struct GraphEntry {
-    GraphKey key;
-    cudaGraphExec_t exec;
-  };
-  std::vector<GraphEntry> graphs_;
-  int parity_ = 0;  // which of the two intensity pyramids currently plays "nextImage"
-  bool use_graphs_ = true;
   void* grid_sync_ = nullptr;  // software grid barrier state of the persistent kernel
   void* dbg_trace_ = nullptr;
   bool time_kernel_ = false;
@@ -168,21 +150,16 @@ class RGBDOdometry {
   double kernel_ms_sum_ = 0;
   int kernel_launches_ = 0;
   bool next_is_last_ = false;  // initAll(): nextDepth pyramid aliases lastDepth (reference quirk)
-  int mode_ = 0;               // 0: one persistent cooperative kernel, 1: per-step kernels (+ CUDA graph)
 
  public:
-  void setUseGraphs(bool v) { use_graphs_ = v; }
-  void setMode(int m) { mode_ = m; }
   // tools only: device buffer of >= 256 u64 receiving a %globaltimer trace of the persistent kernel
   void setDebugTrace(void* dev_u64) { dbg_trace_ = dev_u64; }
   // bench: CUDA-event timing of the dominant kernel (the persistent GN kernel) on its own stream
   void enableKernelTiming(bool on);
   void kernelTiming(double* sum_ms, int* launches, bool reset);
-  int mode() const { return mode_; }
 
  private:
   TrackStats stats_;
-  friend struct DeviceLoopAccess;
 };
 
 }  // namespace cfb

@@ -1,6 +1,6 @@
 // tracker_device.cuh -- per-pixel device functions of the tracker reductions, shared by the
-// stand-alone step kernels (tracker_kernels.cu) and the device-resident Gauss-Newton loop
-// (gn_device.cu).  Arithmetic spec: SURVEY.md Appendix A1-A5 / Core/Cuda/reduce.cu.
+// stand-alone step kernels (tracker_kernels.cu) and the persistent Gauss-Newton kernel
+// (gn_tiled.cu).  Arithmetic spec: SURVEY.md Appendix A1-A5 / Core/Cuda/reduce.cu.
 #pragma once
 #include "tracker_kernels.cuh"
 

@@ -143,10 +143,6 @@ int cfb_odom_get_incremental_transformation(cfb_odom* o, float trans[3], float r
                                             float icpWeight, int pyramid, int fastOdom, int so3,
                                             float* icp_error_map, size_t error_pitch, int force_host_loop,
                                             cfb_track_stats* stats_out, void* stream);
-/* Execution strategy of the default-flag path (no reference equivalent): 0 = one persistent
- * cooperative kernel for the whole SO(3)+GN optimisation (default), 1 = one fused kernel per step
- * replayed as a CUDA graph.  Results are identical. */
-int cfb_odom_set_mode(cfb_odom* o, int mode);
 /* Measurement aid: CUDA events around the dominant tracker kernel on the stream it is launched on;
  * cfb_odom_kernel_timing returns the accumulated milliseconds and launch count (optionally resets). */
 int cfb_odom_enable_kernel_timing(cfb_odom* o, int on);
@@ -234,7 +230,7 @@ int cfb_model_download_map(cfb_model* m, float* dst, size_t capacity_surfels, un
 int cfb_model_upload_map(cfb_model* m, const float* src, unsigned count);
 /* Model::lastCount (Model.h:107) */
 int cfb_model_last_count(cfb_model* m, unsigned* count_out);
-/* the model's tracker (frameToModel), e.g. for cfb_odom_view / cfb_odom_set_mode */
+/* the model's tracker (frameToModel), e.g. for cfb_odom_view */
 cfb_odom* cfb_model_odometry(cfb_model* m);
 /* which: 0 tracker-input vertex+conf (float4) 1 tracker-input normal+radius (float4) 2 tracker-input
  * image (RGBA8) 3 ICP error (f32) | index maps: 4 index (u32) 5 vertConf 6 colorTime 7 normRad (float4)

@@ -10,32 +10,16 @@ for (W, H) in ((640, 480), (1280, 960)):
     case = scenes.room_pair(W, H)
     co = _cuda_odometry(gu, case)
     torch.cuda.synchronize()
-    side = torch.cuda.Stream()
-    for mode, name in ((0, "persistent cooperative kernel"), (1, "per-step kernels, CUDA graph")):
-        co.set_mode(mode)
-        with torch.cuda.stream(side):  # non-default stream -> mode 1 runs as one CUDA graph
-            for _ in range(4):
-                co.track(case["T0"])
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            N = 50
-            e0.record()
-            for _ in range(N):
-                p, st = co.track(case["T0"])
-            e1.record(); torch.cuda.synchronize()
-            print("%dx%d device_loop (%s): %.3f ms/track" % (W, H, name, e0.elapsed_time(e1) / N), flush=True)
-    co.set_mode(1)
-    for host_loop in (False, True):
-        for _ in range(3):
+    for host_loop, name, N in ((False, "persistent cooperative kernel", 50), (True, "host_loop", 20)):
+        for _ in range(4):
             co.track(case["T0"], force_host_loop=host_loop)
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        N = 20
         e0.record()
         for _ in range(N):
             p, st = co.track(case["T0"], force_host_loop=host_loop)
         e1.record(); torch.cuda.synchronize()
-        print("%dx%d %s: %.3f ms/track" % (W, H, "host_loop" if host_loop else "device_loop", e0.elapsed_time(e1) / N), flush=True)
+        print("%dx%d %s: %.3f ms/track" % (W, H, name, e0.elapsed_time(e1) / N), flush=True)
     if orc.ref() is not None and W == 640:
         oo, _ = scenes.oracle_odometry(case)
         for _ in range(2):
